@@ -11,14 +11,17 @@ contiguous slice) and gathers the substitute-edge records of every slice over NC
 output buffer inside every timed step (spg_remove_round_sharded_device; the gather of one size overlaps the
 kernels of the next).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--blankets B] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--blankets B] [--impl reference] [--dump-outputs DIR]
 
-`value`  : device-resident inputs, CUDA events on the library's stream, max over ranks.
+`value`  : device-resident inputs, CUDA events on the library's stream, max over ranks; K timed steps.
 `e2e`    : the same sweep through the host-buffer C-ABI call spg_remove_round (N = 1) /
            spg_remove_round_sharded (N > 1, outputs gathered to rank 0, which holds the graph):
-           pinned host records in, H2D + kernels (+ gather) + D2H inside the timed region.
+           pinned host records in, H2D + kernels (+ gather) + D2H inside the timed region; K timed steps.
 `--impl reference` times the CPU restatement of the reference path (oracle/) on all host threads
 over a bounded sample of the same sweep (the reference itself cannot be built offline).
+`--dump-outputs DIR` writes the output records the last device-resident timed step left in the buffers, decoded, for
+a fixed seeded sample of each size's blankets (at most 64 MB): DIR/n<n>_<field>.npy, float64. The sweep is generated
+from fixed seeds, so two builds run with the same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -61,6 +64,33 @@ def make_sweep(blankets, rank):
         blk["out_off"] = R.out_offsets(6, R.ALG_NFR, R.TOPO_TREE, 1.0, nk)
         sweep.append(blk)
     return sweep
+
+
+DUMP_BYTES = 60 << 20   # --dump-outputs: the arrays of all sizes together (the .npy headers stay within 64 MB)
+DUMP_SEED = 20261020
+
+
+def sample_outputs(dev, sweep):
+    """The device output buffers of every size, decoded for the same seeded sample of blankets in every run: blanket index,
+    status, number of new edges, KLD, and per substitute edge its vertex pair, measurement and information matrix."""
+    import torch
+    n_edges = {d["n"]: R.out_edge_count(R.ALG_NFR, R.TOPO_TREE, 1.0, d["n"] - 1) for d in dev}
+    per_blanket = 8 * sum(4 + ne * (2 + R.pose_words(6) + 36) for ne in n_edges.values())
+    k = DUMP_BYTES // per_blanket
+    rng = np.random.default_rng(DUMP_SEED)
+    arrays = {}
+    for d, blk in zip(dev, sweep):
+        n, B, ne = d["n"], d["B"], n_edges[d["n"]]
+        idx = np.arange(B) if k >= B else np.sort(rng.choice(B, k, replace=False))
+        W = int(blk["out_off"][1] - blk["out_off"][0])   # uniform blankets: one record size per size
+        words = torch.from_numpy(blk["out_off"][idx][:, None] + np.arange(W)).cuda()
+        rec = d["out"][words].cpu().numpy().view(np.uint64)
+        status, pairs, meas, info = R.nfr_uniform_view(rec.reshape(-1), np.arange(len(idx) + 1) * W, 6, n - 1, ne)
+        arrays.update({f"n{n}_blanket": idx, f"n{n}_status": status, f"n{n}_n_new_edges": rec.view(np.int32)[:, 1],
+                       f"n{n}_kld": rec.view(np.float64)[:, 2]})
+        if ne:
+            arrays.update({f"n{n}_pairs": pairs, f"n{n}_meas": meas, f"n{n}_info": info})
+    return {name: np.ascontiguousarray(a, dtype=np.float64) for name, a in arrays.items()}
 
 
 class ClockSampler:
@@ -179,7 +209,13 @@ def main():
     ap.add_argument("--ref-sample", type=int, default=256, help="blankets per size per step for the CPU arms")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--sizes", default=None, help="comma list overriding the size sweep (debug)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed, seeded sample of the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     global SIZES
     if args.sizes:
         SIZES = tuple(int(x) for x in args.sizes.split(","))
@@ -289,6 +325,7 @@ def main():
     barrier()
     dev_ms = ev0.elapsed_time(ev1)  # every step ends with comm_join: ev1 is behind the last gather too
     launches = ctx.launches - launches0
+    dumped = sample_outputs(dev, sweep) if args.dump_outputs and rank == 0 else None  # before the per-size pass below
     # every blanket of the whole sweep must be present and OK in THIS rank's output buffers (own slice from the
     # kernels, the other slices through the gather): status == 0 and n_new_edges == n - 2
     n_dev_ok = 0
@@ -316,7 +353,7 @@ def main():
     clocks = sampler.stop()
 
     # ---- timed: end to end through the host-buffer C ABI ----------------------------------------------
-    e2e_steps = max(1, min(args.steps, 10))   # the same K as the device-resident loop (capped: ~0.13 s per step)
+    e2e_steps = args.steps   # the same K as the device-resident loop (~0.13 s per step)
     shard_info = None
     e2e_modes = {}
     shm = None
@@ -455,6 +492,13 @@ def main():
             nb_total = sum(min(S, blk["B"]) for blk in sweep)
             line["cpu_baseline"] = {"value": nb_total / secs, "unit": UNIT, "cores": cores, "kind": "port",
                                     "sample": f"first {S} blankets of each size of this run's sweep, one blanket per thread"}
+        if dumped is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dumped.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
+            line["dump_outputs"] = {"dir": args.dump_outputs, "arrays": len(dumped),
+                                    "bytes": sum(a.nbytes for a in dumped.values()),
+                                    "blankets_per_size": len(dumped[f"n{SIZES[0]}_blanket"])}
         _emit(line)
     if world > 1:
         dist.barrier()

@@ -146,8 +146,8 @@ __device__ __forceinline__ void publish_panel(const double (&a)[D][D], double *P
 // Sweeps the first nsv vertices of the symmetric matrix held in the blocks (active: vr < nsv): a <- -(A^-1) on the
 // leading block. Pivot j is left in s_piv[j]. Returns false (uniformly) on a non-positive pivot.
 // Per vertex J, two phases with one barrier each:
-//   1. one warp computes the swept panel W_v = P_v B for every other vertex v (P_v = A_vJ and B = A_JJ^-1 were
-//      published during the previous phase 2), two lanes per vertex;
+//   1. the swept panel W_v = P_v B for every other vertex v (P_v = A_vJ and B = A_JJ^-1 were published during the
+//      previous phase 2): one row of one W_v per thread of the CTA (G = 0), or two lanes per vertex of the group;
 //   2. every block (I, L) off the pivot row / column: a -= W_I P_L^T (216 independent DFMAs, 16-byte operand
 //      loads); blocks on the pivot row / column take W; the blocks of vertex J + 1 publish the next panel and
 //      the thread of the next diagonal block inverts it in registers.
@@ -172,7 +172,43 @@ __device__ __forceinline__ bool block_sweep(double (&a)[D][D], double *s_B, doub
         const double *Pc = s_P + (J & 1) * pstride;
         double *Pn = s_P + ((J + 1) & 1) * pstride;
         // ---- phase 1: W_v[q][x] = sum_p P_v[p][x] B[q][p] -----------------------------------------------------------
-        if(tid < LW) {
+        if constexpr(G == 0) {
+            // every thread of the CTA: one row q of one W_v, D independent chains summed over p in the same order as
+            // the lane path below (bit-identical results). Row-major P_v rows and B rows: 16-byte loads and stores.
+            for(int it = tid; it < nsv * D; it += Grp<G>::nt()) {
+                const int v = it / D, q = it % D;
+                if(v == J) continue;
+                const double *Pv = Pc + v * PST, *Bq = B + q * D;
+                double w[D];
+#pragma unroll
+                for(int x = 0; x < D; x++) w[x] = 0;
+#pragma unroll
+                for(int p = 0; p < D; p++) {
+                    const double b = Bq[p];
+                    double px[D];
+                    if constexpr(D % 2 == 0) { // all offsets are even numbers of doubles
+#pragma unroll
+                        for(int x = 0; x < D; x += 2) {
+                            const double2 t = *reinterpret_cast<const double2 *>(Pv + p * D + x);
+                            px[x] = t.x; px[x + 1] = t.y;
+                        }
+                    } else {
+#pragma unroll
+                        for(int x = 0; x < D; x++) px[x] = Pv[p * D + x];
+                    }
+#pragma unroll
+                    for(int x = 0; x < D; x++) w[x] += px[x] * b;
+                }
+                double *Wq = s_W + v * PST + q * D;
+                if constexpr(D % 2 == 0) {
+#pragma unroll
+                    for(int x = 0; x < D; x += 2) *reinterpret_cast<double2 *>(Wq + x) = make_double2(w[x], w[x + 1]);
+                } else {
+#pragma unroll
+                    for(int x = 0; x < D; x++) Wq[x] = w[x];
+                }
+            }
+        } else if(tid < LW) {
 #pragma unroll 1
             for(int v0 = 0; v0 < nsv; v0 += LW / hs) {
                 const int v = v0 + tid / hs, h = tid % hs;

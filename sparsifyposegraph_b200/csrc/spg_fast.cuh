@@ -143,42 +143,56 @@ __device__ __forceinline__ void publish_panel(const double (&a)[D][D], double *P
         for(int x = 0; x < D; x++) Pb[p * D + x] = TRANSPOSED ? a[p][x] : a[x][p];
 }
 
+// Shared-memory panels of one matrix in a block sweep: B x2 (inverted pivot block), P x2 (pivot panel), W (swept
+// panel), piv (its scalar pivots, in sweep order), nsv: vertices swept (0: no such matrix).
+struct SweepSet {
+    double *B, *P, *W, *piv;
+    int nsv;
+};
+
 // Sweeps the first nsv vertices of the symmetric matrix held in the blocks (active: vr < nsv): a <- -(A^-1) on the
-// leading block. Pivot j is left in s_piv[j]. Returns false (uniformly) on a non-positive pivot.
+// leading block. Pivot j is left in piv[j].
 // Per vertex J, two phases with one barrier each:
 //   1. the swept panel W_v = P_v B for every other vertex v (P_v = A_vJ and B = A_JJ^-1 were published during the
 //      previous phase 2): one row of one W_v per thread of the CTA (G = 0), or two lanes per vertex of the group;
 //   2. every block (I, L) off the pivot row / column: a -= W_I P_L^T (216 independent DFMAs, 16-byte operand
 //      loads); blocks on the pivot row / column take W; the blocks of vertex J + 1 publish the next panel and
 //      the thread of the next diagonal block inverts it in registers.
+// G = 0 may sweep two independent matrices s0 and s1 in the same steps (s1.nsv > 0): the thread's block belongs to s1
+// when own1, and phase 1 forms the W rows of both. Every element sees the same operations in the same order as in a
+// sweep of its matrix alone; the step count is the larger nsv, the barriers are shared.
+// Returns (uniformly) bit 0 / bit 1: a non-positive pivot in s0 / s1.
 template <int D, int G>
-__device__ __forceinline__ bool block_sweep(double (&a)[D][D], double *s_B, double *s_P, double *s_W, double *s_piv, int vr, int vc,
-                                            int nsv, bool active, int nkmax) {
+__device__ __forceinline__ int block_sweep(double (&a)[D][D], const SweepSet &s0, const SweepSet &s1, bool own1, int vr, int vc,
+                                           bool active, int nkmax) {
     constexpr int DD = D * D, PST = FastPad<D>::PST;
     constexpr int HS = (D % 2 == 0) ? 2 : 1; // lanes per vertex in phase 1 (nsv <= 16 vertices: otherwise one lane each)
     const int pstride = nkmax * PST;
     const int tid = Grp<G>::tid();
     constexpr int LW = G ? G : 32; // lanes of phase 1
+    const SweepSet m = own1 ? s1 : s0; // the matrix of this thread's block
+    const int nsv = m.nsv, nsteps = max(s0.nsv, s1.nsv);
     bool bad = false;
     if(active) {
-        if(vc == 0 && vr > 0) publish_panel<D, false>(a, s_P + vr * PST);
-        if(vr == 0 && vc == 0) invert_tile<D>(a, s_B, s_piv, bad);
+        if(vc == 0 && vr > 0) publish_panel<D, false>(a, m.P + vr * PST);
+        if(vr == 0 && vc == 0) invert_tile<D>(a, m.B, m.piv, bad);
     }
     Grp<G>::sync();
-    const int hs = (HS * nsv <= LW) ? HS : 1;
+    const int hs = (HS * s0.nsv <= LW) ? HS : 1;
 #pragma unroll 1
-    for(int J = 0; J < nsv; J++) {
-        const double *B = s_B + (J & 1) * DD;
-        const double *Pc = s_P + (J & 1) * pstride;
-        double *Pn = s_P + ((J + 1) & 1) * pstride;
+    for(int J = 0; J < nsteps; J++) {
         // ---- phase 1: W_v[q][x] = sum_p P_v[p][x] B[q][p] -----------------------------------------------------------
         if constexpr(G == 0) {
             // every thread of the CTA: one row q of one W_v, D independent chains summed over p in the same order as
             // the lane path below (bit-identical results). Row-major P_v rows and B rows: 16-byte loads and stores.
-            for(int it = tid; it < nsv * D; it += Grp<G>::nt()) {
-                const int v = it / D, q = it % D;
+            // Rows of s0 first, then those of s1.
+            const int n0 = J < s0.nsv ? s0.nsv * D : 0, n1 = J < s1.nsv ? s1.nsv * D : 0;
+            for(int it = tid; it < n0 + n1; it += Grp<G>::nt()) {
+                const bool second = it >= n0;
+                const int i = second ? it - n0 : it, v = i / D, q = i % D;
                 if(v == J) continue;
-                const double *Pv = Pc + v * PST, *Bq = B + q * D;
+                const SweepSet &S = second ? s1 : s0;
+                const double *Pv = S.P + (J & 1) * pstride + v * PST, *Bq = S.B + (J & 1) * DD + q * D;
                 double w[D];
 #pragma unroll
                 for(int x = 0; x < D; x++) w[x] = 0;
@@ -199,7 +213,7 @@ __device__ __forceinline__ bool block_sweep(double (&a)[D][D], double *s_B, doub
 #pragma unroll
                     for(int x = 0; x < D; x++) w[x] += px[x] * b;
                 }
-                double *Wq = s_W + v * PST + q * D;
+                double *Wq = S.W + v * PST + q * D;
                 if constexpr(D % 2 == 0) {
 #pragma unroll
                     for(int x = 0; x < D; x += 2) *reinterpret_cast<double2 *>(Wq + x) = make_double2(w[x], w[x + 1]);
@@ -208,14 +222,15 @@ __device__ __forceinline__ bool block_sweep(double (&a)[D][D], double *s_B, doub
                     for(int x = 0; x < D; x++) Wq[x] = w[x];
                 }
             }
-        } else if(tid < LW) {
+        } else if(tid < LW) { // G > 0: s0 only
+            const double *B = s0.B + (J & 1) * DD;
 #pragma unroll 1
-            for(int v0 = 0; v0 < nsv; v0 += LW / hs) {
+            for(int v0 = 0; v0 < s0.nsv; v0 += LW / hs) {
                 const int v = v0 + tid / hs, h = tid % hs;
-                if(v < nsv && v != J) {
+                if(v < s0.nsv && v != J) {
                     const int q0 = h * (D / hs), q1 = q0 + D / hs;
-                    const double *Pv = Pc + v * PST;
-                    double *Wv = s_W + v * PST;
+                    const double *Pv = s0.P + (J & 1) * pstride + v * PST;
+                    double *Wv = s0.W + v * PST;
                     if(hs == HS) {
                         double bq[D / HS][D];
 #pragma unroll
@@ -249,21 +264,23 @@ __device__ __forceinline__ bool block_sweep(double (&a)[D][D], double *s_B, doub
         }
         Grp<G>::sync();
         // ---- phase 2 ---------------------------------------------------------------------------------------------
-        if(active && !(vr == J && vc == J)) {
+        if(active && J < nsv && !(vr == J && vc == J)) {
+            const double *Pc = m.P + (J & 1) * pstride;
+            double *Pn = m.P + ((J + 1) & 1) * pstride;
             if(vc == J) { // block (I, J) <- W_I
-                const double *Wb = s_W + vr * PST;
+                const double *Wb = m.W + vr * PST;
 #pragma unroll
                 for(int q = 0; q < D; q++)
 #pragma unroll
                     for(int x = 0; x < D; x++) a[x][q] = Wb[q * D + x];
             } else if(vr == J) { // block (J, L) <- B A_JL = W_L^T
-                const double *Wb = s_W + vc * PST;
+                const double *Wb = m.W + vc * PST;
 #pragma unroll
                 for(int q = 0; q < D; q++)
 #pragma unroll
                     for(int x = 0; x < D; x++) a[q][x] = Wb[q * D + x];
             } else {
-                const double *Wb = s_W + vr * PST, *Pb = Pc + vc * PST;
+                const double *Wb = m.W + vr * PST, *Pb = Pc + vc * PST;
 #pragma unroll
                 for(int p = 0; p < D; p++) {
                     double w[D], q[D];
@@ -289,14 +306,15 @@ __device__ __forceinline__ bool block_sweep(double (&a)[D][D], double *s_B, doub
             }
             if(J + 1 < nsv) {
                 if(vc == J + 1) {
-                    if(vr == J + 1) invert_tile<D>(a, s_B + ((J + 1) & 1) * DD, s_piv + D * (J + 1), bad);
+                    if(vr == J + 1) invert_tile<D>(a, m.B + ((J + 1) & 1) * DD, m.piv + D * (J + 1), bad);
                     else publish_panel<D, false>(a, Pn + vr * PST);
                 } else if(vr == J + 1) publish_panel<D, true>(a, Pn + vc * PST);
             }
         }
         Grp<G>::sync();
     }
-    return Grp<G>::any(bad) == 0;
+    const int bad0 = Grp<G>::any(bad && !own1) ? 1 : 0;
+    return (s1.nsv > 0 && Grp<G>::any(bad && own1)) ? (bad0 | 2) : bad0;
 }
 
 // Cholesky of the diagonal block C_vv = -a held in registers. Lout: column-major D x D, strictly-lower entries of
@@ -378,9 +396,10 @@ __device__ __forceinline__ double schur_logdet_tile(const double (&a)[D][D], con
     return ld_sum;
 }
 
-// shared-memory plan of ONE blanket slot of fast_kernel (doubles; struct FastPlan in spg_plan.h), computed on the host
+// shared-memory plan of ONE blanket slot of fast_kernel (doubles; struct FastPlan in spg_plan.h), computed on the host.
+// fused: the C and G sweeps run side by side (see fast_kernel S3), with a second panel set and a pivot array for C.
 template <int D>
-inline FastPlan fast_plan(int max_nv, int max_e, int max_rec_words, size_t smem_budget_bytes) {
+inline FastPlan fast_plan(int max_nv, int max_e, int max_rec_words, size_t smem_budget_bytes, bool fused) {
     constexpr int PS = PoseStride<D>::value;
     constexpr int JW = 2 * D * D, SW = 4 * D * D, PST = FastPad<D>::PST;
     FastPlan p;
@@ -399,11 +418,13 @@ inline FastPlan fast_plan(int max_nv, int max_e, int max_rec_words, size_t smem_
     // union region.
     //   A (assembly, Schur): record | H00 x2 | H_k0 | Y | J, M of a chunk of edges
     //   B (Schur .. anchored sweep): the Lambda_t blocks [element][tile] | B x2 | P x2 | W   (block sweep panels)
+    //     fused: ... | B2 x2 | P2 x2 | W2 | piv2[kmax]   (panels of the second matrix, pivots of the first)
     //   C (closed form): Jn | Sg | Tm | Bk
     const int rec = (max_rec_words + 1) & ~1;
     const int h0 = 2 * D * D + 2 * D * kmax;
     const int tb = (p.ntiles * D * D + 1) & ~1;
-    const int B = tb + 2 * D * D + 3 * nk * PST;
+    const int set = 2 * D * D + 3 * nk * PST; // one panel set
+    const int B = tb + set + (fused ? set + ((kmax + 1) & ~1) : 0);
     const int C = (nk > 1 ? nk - 1 : 1) * (2 * JW + SW + D * D);
     const int emin = me < 4 ? me : 4;
     int U = rec + h0 + emin * 2 * JW;
@@ -422,6 +443,7 @@ inline FastPlan fast_plan(int max_nv, int max_e, int max_rec_words, size_t smem_
     p.off_B = p.off_U + tb;
     p.off_P = p.off_B + 2 * D * D;
     p.off_W = p.off_P + 2 * nk * PST;
+    p.off_set2 = fused ? set : 0;
     p.total = (p.off_U + U + 1) & ~1;
     return p;
 }
@@ -553,15 +575,16 @@ __global__ void __launch_bounds__(32 * MAXW, G ? 1 : (MAXW <= 4 ? 3 : (D == 6 ? 
         int out_flags = 0;
         if(!refuse) {
             // ---- block of this thread: rows of kept vertex vr, columns of kept vertex vc <= vr ------------------
+            // (fused sweeps: from S3 on, threads ntiles ... ntiles + gtiles - 1 hold the blocks of Lambda_rr, see S3 / S4)
             const int ntiles = nk * (nk + 1) / 2;
-            const bool has_tile = tid < ntiles;
+            bool has_tile = tid < ntiles;
             int vc = 0, vr = 0;
             if(has_tile) {
                 int rem = tid;
                 while(rem >= nk - vc) { rem -= nk - vc; vc++; }
                 vr = vc + rem;
             }
-            const bool diag = has_tile && (vr == vc);
+            bool diag = has_tile && (vr == vc);
             double a[D][D];
 #pragma unroll
             for(int r = 0; r < D; r++)
@@ -769,6 +792,13 @@ __global__ void __launch_bounds__(32 * MAXW, G ? 1 : (MAXW <= 4 ? 3 : (D == 6 ? 
             SPG_FT(2);
             SPG_PHASE(); // 5
             // ---- S3: Chow-Liu tree (pseudo_chow_liu.cpp:33-87) --------------------------------------------------
+            // Fused (the host gave the CTA nkmax^2 threads and a second panel set): the anchored G = Lambda_rr^-1 of S4
+            // is swept in the same block steps as C, on the threads past the C blocks. A failed G pivot is kept in
+            // g_bad and refuses the blanket where the serial order meets it, after guard (ii).
+            const bool fused = pl.off_set2 != 0 && nk > 2;
+            const int gtiles = (nk - 1) * nk / 2;
+            const bool g_own = fused && tid >= ntiles && tid < ntiles + gtiles;
+            bool g_bad = false;
             if(!refuse) {
                 if(nk == 2) {
                     n_out = 1;
@@ -781,7 +811,26 @@ __global__ void __launch_bounds__(32 * MAXW, G ? 1 : (MAXW <= 4 ? 3 : (D == 6 ? 
 #pragma unroll
                         for(int r = 0; r < D; r++) a[r][r] += 1.0;
                     }
-                    if(!block_sweep<D, G>(a, s_B, s_P, s_W, s_piv, vr, vc, nk, has_tile, nkmax)) refuse = true;
+                    SweepSet sc{s_B, s_P, s_W, s_piv, nk}, sg{nullptr, nullptr, nullptr, nullptr, 0};
+                    if(fused) {
+                        double *B2 = s_B + pl.off_set2;
+                        sg = SweepSet{B2, B2 + 2 * DD, B2 + 2 * DD + 2 * nkmax * FastPad<D>::PST, s_piv, nk - 1};
+                        sc.piv = sg.W + nkmax * FastPad<D>::PST; // C's pivots are not used after the sweep
+                        GS::sync(); // the Lambda_t blocks are written
+                        if(g_own) { // block (vr, vc) of the first nk - 1 vertices, loaded from the Lambda_t blocks
+                            int rem = tid - ntiles;
+                            while(rem >= nk - 1 - vc) { rem -= nk - 1 - vc; vc++; }
+                            vr = vc + rem;
+                            const int t = vc * nk - vc * (vc - 1) / 2 + (vr - vc);
+#pragma unroll
+                            for(int r = 0; r < D; r++)
+#pragma unroll
+                                for(int c = 0; c < D; c++) a[r][c] = Tb[(r + c * D) * tstride + t];
+                        }
+                    }
+                    const int swept = block_sweep<D, G>(a, sc, sg, g_own, vr, vc, has_tile || g_own, nkmax);
+                    if(swept & 1) refuse = true;
+                    g_bad = (swept & 2) != 0;
                     if(!refuse) {
                         SPG_FT(3);
                         SPG_PHASE(); // 6
@@ -879,15 +928,31 @@ __global__ void __launch_bounds__(32 * MAXW, G ? 1 : (MAXW <= 4 ? 3 : (D == 6 ? 
                 if(GS::any(bigdiag)) refuse = true;
             }
             if(!refuse) {
-                // G = Lambda_rr^-1 (last kept vertex anchored): reload the blocks and sweep the first nk - 1 vertices
-                const bool act = has_tile && vr < nk - 1;
-                if(has_tile) {
+                // G = Lambda_rr^-1 (last kept vertex anchored): the first nk - 1 vertices swept
+                if(fused) {
+                    // swept in S3. The blocks of G are the g_own threads'; the C threads of the anchored vertex's row
+                    // hold zero blocks for the Sigma scatter, as the serial order below loads them
+                    if(g_bad) refuse = true;
+                    if(!g_own) {
 #pragma unroll
-                    for(int r = 0; r < D; r++)
+                        for(int r = 0; r < D; r++)
 #pragma unroll
-                        for(int c = 0; c < D; c++) a[r][c] = act ? Tb[(r + c * D) * tstride + tid] : 0.0;
+                            for(int c = 0; c < D; c++) a[r][c] = 0.0;
+                    }
+                    has_tile = g_own || (has_tile && vr == nk - 1);
+                    diag = has_tile && vr == vc;
+                } else {
+                    const bool act = has_tile && vr < nk - 1;
+                    if(has_tile) {
+#pragma unroll
+                        for(int r = 0; r < D; r++)
+#pragma unroll
+                            for(int c = 0; c < D; c++) a[r][c] = act ? Tb[(r + c * D) * tstride + tid] : 0.0;
+                    }
+                    const SweepSet sg{s_B, s_P, s_W, s_piv, nk - 1}, none{nullptr, nullptr, nullptr, nullptr, 0};
+                    if(block_sweep<D, G>(a, sg, none, false, vr, vc, act, nkmax)) refuse = true;
                 }
-                if(!block_sweep<D, G>(a, s_B, s_P, s_W, s_piv, vr, vc, nk - 1, act, nkmax)) refuse = true;
+                const bool act = has_tile && vr < nk - 1;
                 if(!refuse) {
                     // guard (i): ||G||_F <= 1e5; log-determinant of Lambda_rr from the pivots
                     double fp = 0;

@@ -19,11 +19,15 @@ spg_status launch_fast(spg_ctx *ctx, spg::KernelParams &kp) {
     // shared memory per blanket slot that still lets the register file's warp / CTA count (MINB) be resident
     constexpr int MINB = G ? (D == 6 ? 12 : 16) : (MAXW <= 4 ? 3 : (D == 6 ? 1 : 2));
     const size_t budget = std::min<size_t>(ctx->smem_optin, (size_t) (228 * 1024) / MINB - 1024) / SPW;
-    const spg::FastPlan pl = spg::fast_plan<D>(kp.max_nv, kp.max_e, kp.max_rec_words, budget);
+    // CTA-wide kernels sweep C and the anchored G side by side (one thread per block of either, nk^2 threads) when the
+    // CTA has room for them: half the serial block steps per blanket
+    const int nk = kp.max_nv > 1 ? kp.max_nv - 1 : 1;
+    const bool fused = G == 0 && nk * nk <= 32 * MAXW;
+    const spg::FastPlan pl = spg::fast_plan<D>(kp.max_nv, kp.max_e, kp.max_rec_words, budget, fused);
     kp.fast = pl;
     const size_t warp_smem = (size_t) pl.total * SPW * sizeof(double);
     const int tiles = spg::fast_tiles(kp.max_nv);
-    int warps = G ? 1 : (tiles + 31) / 32;
+    int warps = G ? 1 : ((fused ? nk * nk : tiles) + 31) / 32;
     if(warp_smem > ctx->smem_optin || warps > MAXW || (G && tiles > G)) return SPG_ERR_UNSUPPORTED;
     if(G) {
         // warps per CTA: a wide round gets as many as the registers (MAXW) and the shared memory allow, one CTA per SM;

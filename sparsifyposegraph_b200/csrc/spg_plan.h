@@ -13,6 +13,7 @@ struct FastPlan {
     int NP, ntiles, chunk;
     int off_pose, off_B, off_P, off_W, off_small, off_U, total;
     int off_h00, off_hk0, off_y, off_jm; // phase A inside the union region U (after the record copy)
+    int off_set2; // C and G sweeps side by side: second panel set at off_B + off_set2 (0: one sweep after the other)
 };
 
 struct KernelParams {

@@ -13,7 +13,7 @@ from sparsifyposegraph_b200 import capi, records as R, synth  # noqa: E402
 
 NAMES = ["load", "assembly", "schur", "cl_chol", "cl_inverse", "cl_blockchol", "cl_mi", "kruskal", "g_chol", "g_inverse",
          "new_jac", "sigma", "x_inv", "glc get_edge+write", "glc marginal", "glc pinv+target"]
-FAST = ["load+poses", "asm: H_k0, H_00", "schur", "C sweep", "MI weights", "kruskal", "G sweep+guards", "closed form",
+FAST = ["load+poses", "asm: H_k0, H_00", "schur", "C (+G) sweep", "MI weights", "kruskal", "G sweep / guards", "closed form",
         "asm: Jacobians", "asm: Omega J", "asm: wait for the other edges", "asm: block gather"] + ["-"] * 4
 sizes = [int(x) for x in sys.argv[1:]] or [5, 16]
 ctx = capi.Context(0)

@@ -617,9 +617,25 @@ __global__ void __launch_bounds__(32 * MAXW, G ? 1 : (MAXW <= 4 ? 3 : (D == 6 ? 
             // ---- S1: assembly. Per chunk of edges (normally all of them): one thread per edge writes J = [Ji Jj] and
             // M = Omega J to shared memory, then every block gathers the edges of its vertex pair in edge order
             // (fixed summation order), and D (k + D) threads gather H_00 and H_k0 from the edges to the removed vertex.
+            // The 4-warp kernel (168 registers, 3 CTAs per SM) keeps its block out of registers across the noinline
+            // edge_jacobians call of a second or later chunk: parked in thread-local memory there (volatile, or the
+            // compiler turns the copy back into registers), and zero before the first chunk. A block live across that
+            // call makes ptxas keep five of its 36 doubles in local memory for the whole kernel, so that every step
+            // of both block sweeps loads and stores them (profiles/r4_sweep_locals.txt). The other variants have 255
+            // registers.
+            constexpr bool park_block = G == 0 && MAXW <= 4;
             const int chunk = pl.chunk;
             for(int e0 = 0; e0 < ne && !refuse; e0 += chunk) {
                 const int ce = min(chunk, ne - e0);
+                [[maybe_unused]] volatile double park[park_block ? D : 1][D];
+                if constexpr(park_block) {
+                    if(e0 > 0) {
+#pragma unroll
+                        for(int r = 0; r < D; r++)
+#pragma unroll
+                            for(int c = 0; c < D; c++) park[r][c] = a[r][c];
+                    }
+                }
                 for(int e = tid; e < ce; e += NT) {
                     const uint64_t *ew = s_rec + r_etab[e0 + e];
                     const int32_t *vi = reinterpret_cast<const int32_t *>(ew + 2);
@@ -652,6 +668,12 @@ __global__ void __launch_bounds__(32 * MAXW, G ? 1 : (MAXW <= 4 ? 3 : (D == 6 ? 
                 }
                 SPG_FT(9);
                 GS::sync();
+                if constexpr(park_block) {
+#pragma unroll
+                    for(int r = 0; r < D; r++)
+#pragma unroll
+                        for(int c = 0; c < D; c++) a[r][c] = e0 > 0 ? park[r][c] : 0.0;
+                }
                 SPG_FT(10);
                 if(e0 == 0) SPG_PHASE(); // 3
                 if(has_tile) {

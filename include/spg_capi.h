@@ -445,12 +445,26 @@ typedef struct {
     int32_t dimensions;
     int32_t terminated;    /* 1: g2o's Terminate (no acceptable step), 0: iteration limit     */
     double chi2_initial, chi2_final, lambda_final;
+    int32_t solver;        /* SPG_SOLVER_DENSE_CHOLESKY or SPG_SOLVER_SPARSE_PCG                */
+    int32_t cg_iterations; /* PCG iterations summed over all trials (0 on the dense path)        */
+    double cg_max_rel_residual; /* largest ||r|| / ||b|| at which a trial's PCG stopped          */
 } spg_optimize_stats;
+#define SPG_SOLVER_DENSE_CHOLESKY 0
+#define SPG_SOLVER_SPARSE_PCG 1
 /*
  * GraphWrapperG2O::optimize (src/graph_wrapper_g2o.cpp:250-269): g2o's OptimizationAlgorithmLevenberg with its
  * default parameters (tau 1e-5, step scales 1/3 .. 2/3, 10 trials after a failure), max_iterations = 50 in the
- * reference, the listed vertices fixed (the reference fixes vertex 0). The linear system is assembled dense in HBM and
- * solved by a blocked Cholesky; the estimates of the graph are updated in place. stats may be NULL.
+ * reference, the listed vertices fixed (the reference fixes vertex 0). The estimates of the graph are updated in place.
+ * stats may be NULL.
+ * The linear system (H + lambda I) x = -g is solved one of two ways, chosen from the problem size and free device
+ * memory alone:
+ *   - dense (SPG_SOLVER_DENSE_CHOLESKY): H assembled dense in HBM and factorised by a blocked Cholesky, whenever
+ *     n^2 * 8 <= 120e9 bytes (n = free dimensions, ~122 k) and the two n x n buffers can be allocated;
+ *   - block-sparse (SPG_SOLVER_SPARSE_PCG): otherwise. H in BSR (D x D blocks of both triangles) and solved by
+ *     conjugate gradients with a block-Jacobi preconditioner (g2o's LinearSolverPCG), from x = 0 to
+ *     ||r|| <= 1e-6 ||b|| or 5000 iterations; a trial that reaches the cap still proposes its step to the rho test.
+ * The environment variable SPG_OPT_DENSE_MAX_DIMS (read on every call) lowers the dense path's limit to that many
+ * dimensions; it exists for tests, like SPG_CHUNK_BYTES.
  */
 spg_status spg_graph_optimize(spg_ctx *ctx, spg_graph *g, const int32_t *fixed_ids, int32_t n_fixed, int32_t max_iterations,
                               spg_optimize_stats *stats);

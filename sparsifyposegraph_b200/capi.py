@@ -66,7 +66,11 @@ class KldTerms(C.Structure):
 
 class OptimizeStats(C.Structure):
     _fields_ = [("iterations", C.c_int32), ("trials", C.c_int32), ("dimensions", C.c_int32), ("terminated", C.c_int32),
-                ("chi2_initial", C.c_double), ("chi2_final", C.c_double), ("lambda_final", C.c_double)]
+                ("chi2_initial", C.c_double), ("chi2_final", C.c_double), ("lambda_final", C.c_double),
+                ("solver", C.c_int32), ("cg_iterations", C.c_int32), ("cg_max_rel_residual", C.c_double)]
+
+
+SOLVER_DENSE_CHOLESKY, SOLVER_SPARSE_PCG = 0, 1   # OptimizeStats.solver
 
 
 class EvaluateInfo(C.Structure):
@@ -374,7 +378,14 @@ class Graph:
         return float(v.value), {f: getattr(t, f) for f, _ in KldTerms._fields_}
 
     def optimize(self, ctx, fixed=(0,), max_iterations=50):
-        """GraphWrapperG2O::optimize (g2o Levenberg-Marquardt over a dense Cholesky on the GPU) -> stats dict."""
+        """GraphWrapperG2O::optimize (g2o Levenberg-Marquardt on the GPU) -> stats dict.
+
+        The linear solve is a dense blocked Cholesky wherever the dense system fits (up to ~122 k free dimensions and
+        enough free device memory for two n x n buffers), and block-sparse preconditioned conjugate gradients beyond
+        that. stats["solver"] says which ran (SOLVER_DENSE_CHOLESKY / SOLVER_SPARSE_PCG); on the sparse path
+        stats["cg_iterations"] sums the CG iterations over all trials and stats["cg_max_rel_residual"] is the worst
+        ||r|| / ||b|| at which a trial stopped. The environment variable SPG_OPT_DENSE_MAX_DIMS, read on every call,
+        lowers the dense limit (for tests)."""
         f = np.ascontiguousarray(list(fixed), dtype=np.int32)
         st = OptimizeStats()
         _check(lib().spg_graph_optimize(ctx.h, self.h, _p(f), len(f), int(max_iterations), C.byref(st)))

@@ -463,6 +463,8 @@ spg_status spg_create(spg_ctx **out, const spg_config *cfg) {
     ctx->smem_optin = prop.sharedMemPerBlockOptin;
     if(const char *e = getenv("SPG_NO_FAST")) ctx->no_fast = atoi(e) != 0;
     if(const char *e = getenv("SPG_CHUNK_BYTES")) ctx->chunk_bytes = std::max<long long>(4096, atoll(e)); // tests: force many chunks
+    // SPG_OPT_DENSE_MAX_DIMS (tests: the optimiser's block-sparse path on small graphs) is read by every
+    // spg_graph_optimize call instead (spg_eval.cu, dense_fits), so it can change after the context exists
     SPG_CUDA(cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
     SPG_CUDA(cudaEventCreate(&ctx->ev0));
     SPG_CUDA(cudaEventCreate(&ctx->ev1));

@@ -6,11 +6,13 @@
 // The reference solves with CHOLMOD on the sparse system and a dense LDLT for the KLD; here the information matrix is
 // assembled dense in HBM (one thread per pose edge, one CTA per GLC factor, fp64 atomics) and factorised with the blocked
 // kernels of spg_dense.cuh — GEMM-shaped FP64 work, thousands of dimensions wide. 180 GB of HBM hold graphs of ~100 k
-// dimensions this way; larger ones are refused (SPG_ERR_UNSUPPORTED), not approximated.
+// dimensions this way. Larger KLDs are refused (SPG_ERR_UNSUPPORTED), not approximated; the optimiser assembles larger
+// systems block-sparse (the same kernels with another addressing policy) and solves them by PCG (spg_sparse.cuh).
 #include <algorithm>
 #include <cmath>
 #include <cstring>
 #include <limits>
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -18,6 +20,7 @@
 #include "spg_dense.cuh"
 #include "spg_glc.cuh"
 #include "spg_host.h"
+#include "spg_sparse.cuh"
 
 namespace {
 
@@ -122,10 +125,31 @@ struct AsmParams {
     double *g;   // gradient sum J^T Omega e (may be NULL)
     double *chi2; // sum e^T Omega e (may be NULL)
     double *scratch;
+    const int32_t *slots;    // BSR: per factor, the slot of its block pair (a, b) at slot_off[edge] + a + b * nv
+    const int64_t *slot_off; // BSR: per factor of the launched kind
+};
+
+// Where the D x D block of H at (vertex a of the factor, vertex b of the factor) lives. pr / pc: first row / column of
+// the two vertices (pos), ia / ib: their places among the factor's nv vertices.
+struct DenseH { // n x n column-major, leading dimension ldh
+    struct Blk { int pr, pc; };
+    template <int D>
+    static __device__ __forceinline__ Blk block(const AsmParams &p, int ei, int nv, int ia, int ib, int pr, int pc) { return {pr, pc}; }
+    template <int D>
+    static __device__ __forceinline__ double *at(const AsmParams &p, Blk b, int r, int c) { return &p.H[(b.pr + r) + (int64_t) (b.pc + c) * p.ldh]; }
+};
+struct BsrH { // one D x D column-major block per slot (spg_sparse.cuh)
+    using Blk = double *;
+    template <int D>
+    static __device__ __forceinline__ Blk block(const AsmParams &p, int ei, int nv, int ia, int ib, int pr, int pc) {
+        return p.H + (int64_t) p.slots[p.slot_off[ei] + ia + ib * nv] * (D * D);
+    }
+    template <int D>
+    static __device__ __forceinline__ double *at(const AsmParams &p, Blk b, int r, int c) { return b + r + c * D; }
 };
 
 // one thread per pose edge: H += J^T Omega J, g += J^T Omega e, chi2 += e^T Omega e
-template <int D>
+template <int D, class A>
 __global__ void __launch_bounds__(64) assemble_pose_edges_kernel(const AsmParams p) {
     constexpr int PS = spg::PoseStride<D>::value, PW = (D == 6) ? 7 : 3;
     double chi = 0.0;
@@ -175,11 +199,12 @@ __global__ void __launch_bounds__(64) assemble_pose_edges_kernel(const AsmParams
                 for(int sb = 0; sb < 2; sb++) {
                     const int pc = sb ? pb : pa;
                     if(pc < 0) continue;
+                    const typename A::Blk blk = A::template block<D>(p, ei, 2, sa, sb, pr, pc);
                     for(int c = 0; c < D; c++)
                         for(int r = 0; r < D; r++) {
                             double s = 0;
                             for(int q = 0; q < D; q++) s += J[sa * D * D + q + r * D] * M[sb * D * D + q + c * D];
-                            atomicAdd(&p.H[(pr + r) + (int64_t) (pc + c) * p.ldh], s);
+                            atomicAdd(A::template at<D>(p, blk, r, c), s);
                         }
                 }
             }
@@ -193,7 +218,7 @@ __global__ void __launch_bounds__(64) assemble_pose_edges_kernel(const AsmParams
 
 // one CTA per GLC factor: J = W * J_reparam (GLCEdge::linearizeOplus, src/glc_edge.cpp:40-49), error = W * r
 // (computeError :28-32), Omega = I
-template <int D>
+template <int D, class A>
 __global__ void __launch_bounds__(64) assemble_glc_edges_kernel(const AsmParams p) {
     constexpr int PS = spg::PoseStride<D>::value, PW = (D == 6) ? 7 : 3, NT = 64;
     const int tid = threadIdx.x;
@@ -259,13 +284,13 @@ __global__ void __launch_bounds__(64) assemble_glc_edges_kernel(const AsmParams 
                 if(pa < 0 || pb < 0) continue;
                 double s = 0;
                 for(int row = 0; row < r; row++) s += Jf[row + (size_t) a * r] * Jf[row + (size_t) b * r];
-                atomicAdd(&p.H[(pa + a % D) + (int64_t) (pb + b % D) * p.ldh], s);
+                atomicAdd(A::template at<D>(p, A::template block<D>(p, ei, nv, a / D, b / D, pa, pb), a % D, b % D), s);
             }
     }
 }
 
 // one CTA per MultiEdgeCorrelated (multi_edge_correlated.hpp:64-140): stacked pose errors and Jacobians, full Omega
-template <int D>
+template <int D, class A>
 __global__ void __launch_bounds__(64) assemble_multi_edges_kernel(const AsmParams p) {
     constexpr int PS = spg::PoseStride<D>::value, PW = (D == 6) ? 7 : 3, NT = 64;
     const int tid = threadIdx.x;
@@ -329,7 +354,7 @@ __global__ void __launch_bounds__(64) assemble_multi_edges_kernel(const AsmParam
                 if(pa < 0 || pb < 0) continue;
                 double s = 0;
                 for(int row = 0; row < rows; row++) s += Jf[row + (size_t) a * rows] * M[row + (size_t) b * rows];
-                atomicAdd(&p.H[(pa + a % D) + (int64_t) (pb + b % D) * p.ldh], s);
+                atomicAdd(A::template at<D>(p, A::template block<D>(p, ei, nv, a / D, b / D, pa, pb), a % D, b % D), s);
             }
     }
 }
@@ -429,11 +454,87 @@ void backward_solve_vec(spg_ctx *ctx, const double *L, int64_t ldl, int n, doubl
     }
 }
 
-struct DevArrays {
-    DevBuf poses, pos, verts, data, pedges, gedges, medges, scratch;
+// Block pattern of H over the free vertices for the sparse path (spg_sparse.cuh): block rows in layout() order, a block
+// for every ordered pair of free vertices of a factor (pose edges 2 x 2; GLC and MULTI nv x nv, since their Omega
+// couples every row) and every diagonal block, both triangles stored.
+struct Bsr {
+    int nb = 0;
+    int64_t nnzb = 0;
+    std::vector<int32_t> rowptr, col, diag; // diag: slot of each row's diagonal block
+    std::vector<int32_t> slots;             // per factor (pose, GLC, then MULTI edges): nv x nv, -1 where a vertex is fixed
+    std::vector<int64_t> slot_off;          // per factor: offset of its table in slots
 };
 
-spg_status upload(spg_ctx *ctx, const DeviceGraph &dg, const std::vector<int32_t> &pos, DevArrays &d) {
+template <class F>
+void for_each_factor(const DeviceGraph &dg, F f) {
+    for(const auto *list : {&dg.pose_edges, &dg.glc_edges, &dg.multi_edges})
+        for(const EdgeRef &e : *list) f(e);
+}
+
+spg_status build_bsr(const DeviceGraph &dg, const std::vector<int32_t> &pos, int n, Bsr &b) {
+    const int D = dg.dim;
+    b.nb = n / D;
+    std::vector<int64_t> start((size_t) b.nb + 1, 0);
+    std::vector<int32_t> rows;
+    auto free_rows = [&](const EdgeRef &e) {
+        rows.clear();
+        for(int q = 0; q < e.nv; q++) {
+            const int pv = pos[dg.verts[e.vert + q]];
+            if(pv >= 0) rows.push_back(pv / D);
+        }
+    };
+    for(int i = 0; i < b.nb; i++) start[i + 1] = 1;
+    for_each_factor(dg, [&](const EdgeRef &e) {
+        free_rows(e);
+        for(int r : rows) start[r + 1] += (int64_t) rows.size();
+    });
+    for(int i = 0; i < b.nb; i++) start[i + 1] += start[i];
+    std::vector<int32_t> cols((size_t) start[b.nb]);
+    std::vector<int64_t> fill(start.begin(), start.end() - 1);
+    for(int i = 0; i < b.nb; i++) cols[fill[i]++] = i;
+    for_each_factor(dg, [&](const EdgeRef &e) {
+        free_rows(e);
+        for(int r : rows)
+            for(int c : rows) cols[fill[r]++] = c;
+    });
+    b.rowptr.assign((size_t) b.nb + 1, 0);
+    b.col.clear();
+    for(int i = 0; i < b.nb; i++) {
+        auto lo = cols.begin() + start[i], hi = cols.begin() + start[i + 1];
+        std::sort(lo, hi);
+        b.col.insert(b.col.end(), lo, std::unique(lo, hi));
+        if(b.col.size() > (size_t) std::numeric_limits<int32_t>::max()) {
+            spg_set_err("spg_graph_optimize: block-sparse system has more than 2^31 blocks");
+            return SPG_ERR_UNSUPPORTED;
+        }
+        b.rowptr[i + 1] = (int32_t) b.col.size();
+    }
+    b.nnzb = (int64_t) b.col.size();
+    auto slot_of = [&](int r, int c) {
+        const auto lo = b.col.begin() + b.rowptr[r], hi = b.col.begin() + b.rowptr[r + 1];
+        return (int32_t) (std::lower_bound(lo, hi, c) - b.col.begin());
+    };
+    b.diag.resize((size_t) b.nb);
+    for(int i = 0; i < b.nb; i++) b.diag[i] = slot_of(i, i);
+    b.slots.clear();
+    b.slot_off.clear();
+    for_each_factor(dg, [&](const EdgeRef &e) {
+        b.slot_off.push_back((int64_t) b.slots.size());
+        for(int ib = 0; ib < e.nv; ib++)
+            for(int ia = 0; ia < e.nv; ia++) {
+                const int pa = pos[dg.verts[e.vert + ia]], pb = pos[dg.verts[e.vert + ib]];
+                b.slots.push_back(pa >= 0 && pb >= 0 ? slot_of(pa / D, pb / D) : -1);
+            }
+    });
+    return SPG_OK;
+}
+
+struct DevArrays {
+    DevBuf poses, pos, verts, data, pedges, gedges, medges, scratch, slots, slot_off;
+};
+
+// bsr: the slot tables of the sparse path (NULL: dense H)
+spg_status upload(spg_ctx *ctx, const DeviceGraph &dg, const std::vector<int32_t> &pos, DevArrays &d, const Bsr *bsr = nullptr) {
     cudaStream_t st = ctx->stream;
     SPG_CUDA(d.poses.reserve(dg.poses.size() * 8 + 8));
     SPG_CUDA(d.pos.reserve(pos.size() * 4 + 8));
@@ -453,16 +554,25 @@ spg_status upload(spg_ctx *ctx, const DeviceGraph &dg, const std::vector<int32_t
         SPG_CUDA(cudaMemcpyAsync(d.gedges.p, dg.glc_edges.data(), dg.glc_edges.size() * sizeof(EdgeRef), cudaMemcpyHostToDevice, st));
     if(!dg.multi_edges.empty())
         SPG_CUDA(cudaMemcpyAsync(d.medges.p, dg.multi_edges.data(), dg.multi_edges.size() * sizeof(EdgeRef), cudaMemcpyHostToDevice, st));
+    if(bsr) {
+        SPG_CUDA(d.slots.reserve(bsr->slots.size() * 4 + 8));
+        SPG_CUDA(d.slot_off.reserve(bsr->slot_off.size() * 8 + 8));
+        SPG_CUDA(cudaMemcpyAsync(d.slots.p, bsr->slots.data(), bsr->slots.size() * 4, cudaMemcpyHostToDevice, st));
+        SPG_CUDA(cudaMemcpyAsync(d.slot_off.p, bsr->slot_off.data(), bsr->slot_off.size() * 8, cudaMemcpyHostToDevice, st));
+    }
     return SPG_OK;
 }
 void release(DevArrays &d) {
-    for(DevBuf *b : {&d.poses, &d.pos, &d.verts, &d.data, &d.pedges, &d.gedges, &d.medges, &d.scratch}) b->release();
+    for(DevBuf *b : {&d.poses, &d.pos, &d.verts, &d.data, &d.pedges, &d.gedges, &d.medges, &d.scratch, &d.slots, &d.slot_off}) b->release();
 }
 
-// H (n x n, zeroed here when given), g (n, zeroed), chi2 (1, zeroed) of the graph at the uploaded poses
-spg_status assemble(spg_ctx *ctx, const DeviceGraph &dg, DevArrays &d, int n, double *H, int64_t ldh, double *g, double *chi2) {
+// H (zeroed here when given), g (n, zeroed), chi2 (1, zeroed) of the graph at the uploaded poses. H is the n x n dense
+// matrix of leading dimension ldh, or with bsr_blocks > 0 the values of that many BSR blocks (slot tables uploaded).
+spg_status assemble(spg_ctx *ctx, const DeviceGraph &dg, DevArrays &d, int n, double *H, int64_t ldh, double *g, double *chi2,
+                    int64_t bsr_blocks = 0) {
     cudaStream_t st = ctx->stream;
-    if(H) SPG_CUDA(cudaMemsetAsync(H, 0, (size_t) ldh * n * 8, st));
+    const bool bsr = bsr_blocks > 0;
+    if(H) SPG_CUDA(cudaMemsetAsync(H, 0, bsr ? (size_t) bsr_blocks * dg.dim * dg.dim * 8 : (size_t) ldh * n * 8, st));
     if(g) SPG_CUDA(cudaMemsetAsync(g, 0, (size_t) n * 8, st));
     if(chi2) SPG_CUDA(cudaMemsetAsync(chi2, 0, 8, st));
     AsmParams p{};
@@ -475,30 +585,41 @@ spg_status assemble(spg_ctx *ctx, const DeviceGraph &dg, DevArrays &d, int n, do
     p.g = g;
     p.chi2 = chi2;
     p.scratch = static_cast<double *>(d.scratch.p);
+    p.slots = static_cast<const int32_t *>(d.slots.p);
+    const int64_t *slot_off = static_cast<const int64_t *>(d.slot_off.p);
+#define SPG_ASM_LAUNCH(kernel, blocks)                                       \
+    do {                                                                     \
+        if(bsr) {                                                            \
+            if(dg.dim == 6) kernel<6, BsrH><<<blocks, 64, 0, st>>>(p);       \
+            else kernel<3, BsrH><<<blocks, 64, 0, st>>>(p);                  \
+        } else {                                                             \
+            if(dg.dim == 6) kernel<6, DenseH><<<blocks, 64, 0, st>>>(p);     \
+            else kernel<3, DenseH><<<blocks, 64, 0, st>>>(p);                \
+        }                                                                    \
+        ctx->launches++;                                                     \
+    } while(0)
     if(!dg.pose_edges.empty()) {
         p.edges = static_cast<const EdgeRef *>(d.pedges.p);
         p.n_edges = (int) dg.pose_edges.size();
+        p.slot_off = slot_off;
         const int blocks = std::min<int>((p.n_edges + 63) / 64, ctx->sm_count * 16);
-        if(dg.dim == 6) assemble_pose_edges_kernel<6><<<blocks, 64, 0, st>>>(p);
-        else assemble_pose_edges_kernel<3><<<blocks, 64, 0, st>>>(p);
-        ctx->launches++;
+        SPG_ASM_LAUNCH(assemble_pose_edges_kernel, blocks);
     }
     if(!dg.glc_edges.empty()) {
         p.edges = static_cast<const EdgeRef *>(d.gedges.p);
         p.n_edges = (int) dg.glc_edges.size();
+        p.slot_off = slot_off ? slot_off + dg.pose_edges.size() : nullptr;
         const int blocks = std::min<int>(p.n_edges, ctx->sm_count * 16);
-        if(dg.dim == 6) assemble_glc_edges_kernel<6><<<blocks, 64, 0, st>>>(p);
-        else assemble_glc_edges_kernel<3><<<blocks, 64, 0, st>>>(p);
-        ctx->launches++;
+        SPG_ASM_LAUNCH(assemble_glc_edges_kernel, blocks);
     }
     if(!dg.multi_edges.empty()) {
         p.edges = static_cast<const EdgeRef *>(d.medges.p);
         p.n_edges = (int) dg.multi_edges.size();
+        p.slot_off = slot_off ? slot_off + dg.pose_edges.size() + dg.glc_edges.size() : nullptr;
         const int blocks = std::min<int>(p.n_edges, ctx->sm_count * 16);
-        if(dg.dim == 6) assemble_multi_edges_kernel<6><<<blocks, 64, 0, st>>>(p);
-        else assemble_multi_edges_kernel<3><<<blocks, 64, 0, st>>>(p);
-        ctx->launches++;
+        SPG_ASM_LAUNCH(assemble_multi_edges_kernel, blocks);
     }
+#undef SPG_ASM_LAUNCH
     SPG_CUDA(cudaGetLastError());
     return SPG_OK;
 }
@@ -537,6 +658,257 @@ void oplus_flat(int dim, double *pose, const double *d) {
     double out[7];
     spg::poseCompose(6, pose, q, out);
     std::memcpy(pose, out, sizeof(out));
+}
+
+// ---- spg_graph_optimize: one Levenberg-Marquardt driver over two ways of storing and solving the system ----------------
+// The steps that depend on the storage of H. g (n doubles) and sc ([0] chi2, [1] max diagonal) belong to the driver.
+struct LinearSystem {
+    int64_t cg_iterations = 0;
+    double cg_max_rel_residual = 0;
+    virtual ~LinearSystem() = default;
+    // H, g and chi2 at the uploaded poses
+    virtual spg_status build(double *g, double *chi2) = 0;
+    virtual spg_status max_diag(double *out) = 0;
+    // (H + lambda I) x = -g into hx; *ok = false when H + lambda I is not positive definite
+    virtual spg_status solve(double lambda, const double *g, const std::vector<double> &hg, std::vector<double> &hx, bool *ok) = 0;
+};
+
+// H dense in HBM, blocked Cholesky + forward / backward substitution (spg_dense.cuh)
+struct DenseSystem : LinearSystem {
+    spg_ctx *ctx;
+    const DeviceGraph &dg;
+    DevArrays &arr;
+    const int n;
+    DevBuf dH, dwork, dx, dflag; // H, H + lambda I and its factor, x, Cholesky flag
+    DenseSystem(spg_ctx *c, const DeviceGraph &d, DevArrays &a, int n_) : ctx(c), dg(d), arr(a), n(n_) {}
+    ~DenseSystem() override {
+        for(DevBuf *b : {&dH, &dwork, &dx, &dflag}) b->release();
+    }
+    cudaError_t reserve() {
+        const size_t nn = (size_t) std::max(n, 1);
+        cudaError_t e = dH.reserve(nn * nn * 8);
+        if(e == cudaSuccess) e = dx.reserve(nn * 8);
+        if(e == cudaSuccess) e = dflag.reserve(8);
+        if(e == cudaSuccess) e = dwork.reserve(nn * nn * 8);
+        return e;
+    }
+    spg_status build(double *g, double *chi2) override {
+        return assemble(ctx, dg, arr, n, static_cast<double *>(dH.p), n, g, chi2);
+    }
+    spg_status max_diag(double *out) override {
+        max_diag_kernel<<<1, 1024, 0, ctx->stream>>>(static_cast<double *>(dH.p), n, n, out);
+        return SPG_OK;
+    }
+    spg_status solve(double lambda, const double *, const std::vector<double> &hg, std::vector<double> &hx, bool *ok) override {
+        cudaStream_t st = ctx->stream;
+        double *Wk = static_cast<double *>(dwork.p), *x = static_cast<double *>(dx.p);
+        int *flag = static_cast<int *>(dflag.p);
+        SPG_CUDA(cudaMemcpyAsync(Wk, dH.p, (size_t) n * n * 8, cudaMemcpyDeviceToDevice, st));
+        add_diag_kernel<<<(n + 255) / 256, 256, 0, st>>>(Wk, n, n, lambda);
+        SPG_CUDA(cudaMemsetAsync(flag, 0, 4, st));
+        cholesky_partial(ctx, Wk, n, n, n, nullptr, flag);
+        for(int q = 0; q < n; q++) hx[q] = -hg[q];
+        SPG_CUDA(cudaMemcpyAsync(x, hx.data(), (size_t) n * 8, cudaMemcpyHostToDevice, st));
+        forward_solve(ctx, Wk, n, n, x, n, 1);
+        backward_solve_vec(ctx, Wk, n, n, x);
+        int hflag = 0;
+        SPG_CUDA(cudaMemcpyAsync(hx.data(), x, (size_t) n * 8, cudaMemcpyDeviceToHost, st));
+        SPG_CUDA(cudaMemcpyAsync(&hflag, flag, 4, cudaMemcpyDeviceToHost, st));
+        SPG_CUDA(cudaStreamSynchronize(st));
+        *ok = hflag == 0;
+        return SPG_OK;
+    }
+};
+
+// H block-sparse (BSR, both triangles), block-Jacobi PCG (spg_sparse.cuh)
+struct SparseSystem : LinearSystem {
+    spg_ctx *ctx;
+    const DeviceGraph &dg;
+    DevArrays &arr;
+    const Bsr &bsr;
+    const int n, nb, grid_spmv, grid_rows;
+    DevBuf dvals, drowptr, dcol, ddiag, dminv, dx, dr, dz, dp0, dp1, dq, dpart, dstate;
+    SparseSystem(spg_ctx *c, const DeviceGraph &d, DevArrays &a, const Bsr &b, int n_)
+        : ctx(c), dg(d), arr(a), bsr(b), n(n_), nb(b.nb),
+          grid_spmv(std::max(1, std::min((b.nb + 7) / 8, c->sm_count * spg::PCG_CTAS_PER_SM))),
+          grid_rows(std::max(1, std::min((b.nb + 255) / 256, c->sm_count * spg::PCG_CTAS_PER_SM))) {}
+    ~SparseSystem() override {
+        for(DevBuf *b : {&dvals, &drowptr, &dcol, &ddiag, &dminv, &dx, &dr, &dz, &dp0, &dp1, &dq, &dpart, &dstate}) b->release();
+    }
+    spg_status reserve() {
+        cudaStream_t st = ctx->stream;
+        const int D = dg.dim;
+        const size_t vec = (size_t) n * 8 + 8, part = (size_t) 3 * ctx->sm_count * spg::PCG_CTAS_PER_SM * 8;
+        SPG_CUDA(dvals.reserve((size_t) bsr.nnzb * D * D * 8 + 8));
+        SPG_CUDA(drowptr.reserve(bsr.rowptr.size() * 4 + 8));
+        SPG_CUDA(dcol.reserve(bsr.col.size() * 4 + 8));
+        SPG_CUDA(ddiag.reserve(bsr.diag.size() * 4 + 8));
+        SPG_CUDA(dminv.reserve((size_t) nb * D * D * 8 + 8));
+        for(DevBuf *b : {&dx, &dr, &dz, &dp0, &dp1, &dq}) SPG_CUDA(b->reserve(vec));
+        SPG_CUDA(dpart.reserve(part));
+        SPG_CUDA(dstate.reserve(sizeof(spg::PcgState)));
+        SPG_CUDA(cudaMemcpyAsync(drowptr.p, bsr.rowptr.data(), bsr.rowptr.size() * 4, cudaMemcpyHostToDevice, st));
+        SPG_CUDA(cudaMemcpyAsync(dcol.p, bsr.col.data(), bsr.col.size() * 4, cudaMemcpyHostToDevice, st));
+        SPG_CUDA(cudaMemcpyAsync(ddiag.p, bsr.diag.data(), bsr.diag.size() * 4, cudaMemcpyHostToDevice, st));
+        return SPG_OK;
+    }
+    spg_status build(double *g, double *chi2) override {
+        return assemble(ctx, dg, arr, n, static_cast<double *>(dvals.p), 0, g, chi2, std::max<int64_t>(bsr.nnzb, 1));
+    }
+    spg_status max_diag(double *out) override {
+        const double *v = static_cast<const double *>(dvals.p);
+        const int32_t *dd = static_cast<const int32_t *>(ddiag.p);
+        if(dg.dim == 6) spg::bsr_max_diag_kernel<6><<<1, 1024, 0, ctx->stream>>>(v, dd, nb, out);
+        else spg::bsr_max_diag_kernel<3><<<1, 1024, 0, ctx->stream>>>(v, dd, nb, out);
+        return SPG_OK;
+    }
+    spg_status solve(double lambda, const double *g, const std::vector<double> &, std::vector<double> &hx, bool *ok) override {
+        return dg.dim == 6 ? pcg<6>(lambda, g, hx, ok) : pcg<3>(lambda, g, hx, ok);
+    }
+    template <int D>
+    spg_status pcg(double lambda, const double *g, std::vector<double> &hx, bool *ok) {
+        cudaStream_t st = ctx->stream;
+        const double *vals = static_cast<const double *>(dvals.p);
+        const int32_t *rowptr = static_cast<const int32_t *>(drowptr.p), *col = static_cast<const int32_t *>(dcol.p);
+        double *Minv = static_cast<double *>(dminv.p), *x = static_cast<double *>(dx.p), *r = static_cast<double *>(dr.p);
+        double *z = static_cast<double *>(dz.p), *q = static_cast<double *>(dq.p);
+        double *pq = static_cast<double *>(dpart.p), *prz = pq + ctx->sm_count * spg::PCG_CTAS_PER_SM;
+        double *prr = prz + ctx->sm_count * spg::PCG_CTAS_PER_SM;
+        double *pa = static_cast<double *>(dp0.p), *pb = static_cast<double *>(dp1.p);
+        spg::PcgState *state = static_cast<spg::PcgState *>(dstate.p);
+        SPG_CUDA(cudaMemsetAsync(state, 0, sizeof(spg::PcgState), st));
+        SPG_CUDA(cudaMemsetAsync(pa, 0, (size_t) n * 8, st)); // p_0 = z_0 + 0 * pa
+        spg::bsr_block_jacobi_kernel<D><<<grid_rows, 256, 0, st>>>(vals, static_cast<const int32_t *>(ddiag.p), nb, lambda, Minv, state);
+        spg::pcg_update_kernel<D><<<grid_rows, 256, 0, st>>>(nb, true, Minv, g, pa, q, x, r, z, state, prz, prr);
+        spg::pcg_beta_kernel<<<1, 1024, 0, st>>>(prz, prr, grid_rows, true, spg::PCG_TOL, spg::PCG_MAX_ITERS, state);
+        ctx->launches += 3;
+        spg::PcgState h{};
+        for(;;) {
+            for(int k = 0; k < spg::PCG_POLL; k++) {
+                spg::pcg_spmv_dot_kernel<D><<<grid_spmv, 256, 0, st>>>(nb, rowptr, col, vals, lambda, z, pa, pb, q, state, pq);
+                spg::pcg_alpha_kernel<<<1, 1024, 0, st>>>(pq, grid_spmv, state);
+                spg::pcg_update_kernel<D><<<grid_rows, 256, 0, st>>>(nb, false, Minv, g, pb, q, x, r, z, state, prz, prr);
+                spg::pcg_beta_kernel<<<1, 1024, 0, st>>>(prz, prr, grid_rows, false, spg::PCG_TOL, spg::PCG_MAX_ITERS, state);
+                std::swap(pa, pb);
+            }
+            ctx->launches += 4 * spg::PCG_POLL;
+            SPG_CUDA(cudaMemcpyAsync(&h, state, sizeof(h), cudaMemcpyDeviceToHost, st));
+            SPG_CUDA(cudaStreamSynchronize(st));
+            if(h.done) break;
+        }
+        SPG_CUDA(cudaGetLastError());
+        SPG_CUDA(cudaMemcpyAsync(hx.data(), x, (size_t) n * 8, cudaMemcpyDeviceToHost, st));
+        SPG_CUDA(cudaStreamSynchronize(st));
+        cg_iterations += h.iters;
+        cg_max_rel_residual = std::max(cg_max_rel_residual, h.rel);
+        *ok = !h.bad;
+        if(!*ok) std::fill(hx.begin(), hx.end(), 0.0); // the trial is rejected; keep computeScale finite
+        return SPG_OK;
+    }
+};
+
+struct LmResult {
+    int iterations = 0, trials = 0;
+    bool terminated = false;
+    double chi2_initial = 0, chi2 = 0, lambda = 0;
+};
+
+// GraphWrapperG2O::optimize (:250-269) with g2o's OptimizationAlgorithmLevenberg (default parameters) on the poses of
+// dg, which are uploaded in arr and updated in both. g: n doubles, sc: 2 doubles of device scratch.
+spg_status levenberg_marquardt(spg_ctx *ctx, DeviceGraph &dg, DevArrays &arr, const std::vector<int32_t> &pos, int n,
+                               int max_iterations, LinearSystem &sys, double *g, double *sc, LmResult &res) {
+    cudaStream_t st = ctx->stream;
+    auto push_poses = [&]() -> cudaError_t {
+        return cudaMemcpyAsync(arr.poses.p, dg.poses.data(), dg.poses.size() * 8, cudaMemcpyHostToDevice, st);
+    };
+    auto chi2_only = [&](double *out) -> spg_status {
+        spg_status s = assemble(ctx, dg, arr, n, nullptr, n, nullptr, sc);
+        if(s != SPG_OK) return s;
+        SPG_CUDA(cudaMemcpyAsync(out, sc, 8, cudaMemcpyDeviceToHost, st));
+        SPG_CUDA(cudaStreamSynchronize(st));
+        return SPG_OK;
+    };
+#define SPG_TRY(call)           \
+    do {                        \
+        spg_status s_ = (call); \
+        if(s_ != SPG_OK) return s_; \
+    } while(0)
+    const size_t nn = (size_t) std::max(n, 1);
+    std::vector<double> hx(nn), hg(nn), saved;
+    double lambda = 0, ni = 2, chi = 0;
+    int iters = 0, trials_total = 0;
+    bool terminated = false;
+    SPG_TRY(chi2_only(&chi));
+    const double chi_initial = chi;
+    for(int it = 0; it < max_iterations && n > 0 && !terminated; it++) {
+        // buildSystem at the current estimates
+        SPG_TRY(sys.build(g, sc));
+        if(it == 0) { // computeLambdaInit: tau * max diagonal entry, tau = 1e-5
+            SPG_TRY(sys.max_diag(sc + 1));
+            double md = 0;
+            SPG_CUDA(cudaMemcpyAsync(&md, sc + 1, 8, cudaMemcpyDeviceToHost, st));
+            SPG_CUDA(cudaStreamSynchronize(st));
+            lambda = 1e-5 * md;
+            ni = 2;
+        }
+        SPG_CUDA(cudaMemcpyAsync(hg.data(), g, (size_t) n * 8, cudaMemcpyDeviceToHost, st));
+        double rho = 0;
+        int qmax = 0;
+        saved = dg.poses;
+        do {
+            // (H + lambda I) x = -g   [g2o: b = -J^T Omega e]
+            bool ok2 = false;
+            SPG_TRY(sys.solve(lambda, g, hg, hx, &ok2));
+            // update (push / oplus)
+            if(ok2)
+                for(int v = 0; v < dg.nV; v++)
+                    if(pos[v] >= 0) oplus_flat(dg.dim, &dg.poses[(size_t) v * dg.P], &hx[pos[v]]);
+            SPG_CUDA(push_poses());
+            double tempChi = 0;
+            SPG_TRY(chi2_only(&tempChi));
+            if(!ok2) tempChi = std::numeric_limits<double>::max();
+            rho = chi - tempChi;
+            double scale = 0; // computeScale: sum x_j (lambda x_j + b_j), b = -g
+            for(int q = 0; q < n; q++) scale += hx[q] * (lambda * hx[q] - hg[q]);
+            scale += 1e-3;
+            rho /= scale;
+            if(rho > 0 && std::isfinite(tempChi)) { // last step was good
+                double alpha = 1.0 - std::pow(2 * rho - 1, 3);
+                alpha = std::min(alpha, 2.0 / 3.0);
+                lambda *= std::max(1.0 / 3.0, alpha);
+                ni = 2;
+                chi = tempChi;
+            } else {
+                lambda *= ni;
+                ni *= 2;
+                dg.poses = saved; // pop
+                SPG_CUDA(push_poses());
+                if(!std::isfinite(lambda)) break;
+            }
+            qmax++;
+            trials_total++;
+        } while(rho < 0 && qmax < 10);
+        iters++;
+        if(qmax == 10 || rho == 0 || !std::isfinite(lambda)) terminated = true;
+    }
+#undef SPG_TRY
+    SPG_CUDA(cudaStreamSynchronize(st));
+    res.iterations = iters;
+    res.trials = trials_total;
+    res.terminated = terminated;
+    res.chi2_initial = chi_initial;
+    res.chi2 = chi;
+    res.lambda = lambda;
+    return SPG_OK;
+}
+
+// Largest system the dense path takes: two n x n buffers of 8-byte words, 120 GB for H, as before the sparse path. The
+// environment variable SPG_OPT_DENSE_MAX_DIMS lowers it (tests: the sparse path on graphs the dense path also solves);
+// read on every call so it can be set after the library is loaded.
+bool dense_fits(int n) {
+    if((double) n * n * 8 > 120e9) return false;
+    const char *e = getenv("SPG_OPT_DENSE_MAX_DIMS");
+    return !(e && *e && n > atoll(e));
 }
 
 } // namespace
@@ -699,8 +1071,9 @@ spg_status spg_graph_kld(spg_ctx *ctx, const spg_graph *full, const spg_graph *s
     return SPG_OK;
 }
 
-// GraphWrapperG2O::optimize (:250-269) with g2o's OptimizationAlgorithmLevenberg (default parameters) over a dense
-// Cholesky. fixed_ids: the vertices held fixed (the reference fixes vertex 0; chi2(other) fixes other's vertices).
+// GraphWrapperG2O::optimize (:250-269) with g2o's OptimizationAlgorithmLevenberg (default parameters). fixed_ids: the
+// vertices held fixed (the reference fixes vertex 0; chi2(other) fixes other's vertices). Dense Cholesky wherever the
+// dense system fits; block-sparse PCG beyond that.
 spg_status spg_graph_optimize(spg_ctx *ctx, spg_graph *gr, const int32_t *fixed_ids, int32_t n_fixed, int32_t max_iterations,
                               spg_optimize_stats *stats) {
     if(!ctx || !gr || n_fixed < 0 || (n_fixed > 0 && !fixed_ids) || max_iterations < 0) {
@@ -720,15 +1093,15 @@ spg_status spg_graph_optimize(spg_ctx *ctx, spg_graph *gr, const int32_t *fixed_
     std::vector<int32_t> pos;
     const int n = layout(dg, fixed, nullptr, pos, nullptr);
     if(stats) *stats = spg_optimize_stats{};
-    if((double) n * n * 8 > 120e9) {
-        spg_set_err("spg_graph_optimize: dense system of " + std::to_string(n) + " dimensions does not fit");
-        return SPG_ERR_UNSUPPORTED;
-    }
-    cudaStream_t st = ctx->stream;
-    DevBuf dH, dg_, dx, dsc, dwork;
+    DevBuf dg_, dsc;
     DevArrays arr;
+    Bsr bsr;
+    std::unique_ptr<DenseSystem> dense;
+    std::unique_ptr<SparseSystem> sparse;
     auto cleanup = [&] {
-        for(DevBuf *b : {&dH, &dg_, &dx, &dsc, &dwork}) b->release();
+        dense.reset();
+        sparse.reset();
+        for(DevBuf *b : {&dg_, &dsc}) b->release();
         release(arr);
     };
 #define SPG_CUDA_C(call)                                                            \
@@ -748,96 +1121,32 @@ spg_status spg_graph_optimize(spg_ctx *ctx, spg_graph *gr, const int32_t *fixed_
             return s_;                   \
         }                                \
     } while(0)
-    const int nn = std::max(n, 1);
-    SPG_CUDA_C(dH.reserve((size_t) nn * nn * 8));
-    SPG_CUDA_C(dg_.reserve((size_t) nn * 8));
-    SPG_CUDA_C(dx.reserve((size_t) nn * 8));
-    SPG_CUDA_C(dsc.reserve(64));
-    SPG_CUDA_C(dwork.reserve((size_t) nn * nn * 8)); // H + lambda I and its factor
-    double *Wk = static_cast<double *>(dwork.p);
-    double *H = static_cast<double *>(dH.p), *g = static_cast<double *>(dg_.p), *x = static_cast<double *>(dx.p);
-    double *sc = static_cast<double *>(dsc.p); // [0] chi2 [1] max diag [2] logdet (unused), flag at +24
-    int *flag = reinterpret_cast<int *>(sc + 3);
-    SPG_TRY(upload(ctx, dg, pos, arr));
-    auto push_poses = [&]() -> cudaError_t {
-        return cudaMemcpyAsync(arr.poses.p, dg.poses.data(), dg.poses.size() * 8, cudaMemcpyHostToDevice, st);
-    };
-    auto chi2_only = [&](double *out) -> spg_status {
-        spg_status s = assemble(ctx, dg, arr, n, nullptr, n, nullptr, sc);
-        if(s != SPG_OK) return s;
-        SPG_CUDA(cudaMemcpyAsync(out, sc, 8, cudaMemcpyDeviceToHost, st));
-        SPG_CUDA(cudaStreamSynchronize(st));
-        return SPG_OK;
-    };
-    std::vector<double> hx((size_t) nn), hg((size_t) nn), saved;
-    double lambda = 0, ni = 2, chi = 0;
-    int iters = 0, trials_total = 0;
-    bool terminated = false;
-    SPG_TRY(chi2_only(&chi));
-    const double chi_initial = chi;
-    for(int it = 0; it < max_iterations && n > 0 && !terminated; it++) {
-        // buildSystem at the current estimates
-        SPG_TRY(assemble(ctx, dg, arr, n, H, n, g, sc));
-        if(it == 0) { // computeLambdaInit: tau * max diagonal entry, tau = 1e-5
-            max_diag_kernel<<<1, 1024, 0, st>>>(H, n, n, sc + 1);
-            double md = 0;
-            SPG_CUDA_C(cudaMemcpyAsync(&md, sc + 1, 8, cudaMemcpyDeviceToHost, st));
-            SPG_CUDA_C(cudaStreamSynchronize(st));
-            lambda = 1e-5 * md;
-            ni = 2;
+    if(dense_fits(n)) {
+        dense.reset(new DenseSystem(ctx, dg, arr, n));
+        const cudaError_t e = dense->reserve();
+        if(e == cudaErrorMemoryAllocation) { // not enough free HBM for the two dense buffers: go sparse
+            cudaGetLastError();
+            dense.reset();
+        } else {
+            SPG_CUDA_C(e);
         }
-        SPG_CUDA_C(cudaMemcpyAsync(hg.data(), g, (size_t) n * 8, cudaMemcpyDeviceToHost, st));
-        double rho = 0;
-        int qmax = 0;
-        saved = dg.poses;
-        do {
-            // (H + lambda I) x = -g   [g2o: b = -J^T Omega e]
-            SPG_CUDA_C(cudaMemcpyAsync(Wk, H, (size_t) n * n * 8, cudaMemcpyDeviceToDevice, st));
-            add_diag_kernel<<<(n + 255) / 256, 256, 0, st>>>(Wk, n, n, lambda);
-            SPG_CUDA_C(cudaMemsetAsync(flag, 0, 4, st));
-            cholesky_partial(ctx, Wk, n, n, n, nullptr, flag);
-            for(int q = 0; q < n; q++) hx[q] = -hg[q];
-            SPG_CUDA_C(cudaMemcpyAsync(x, hx.data(), (size_t) n * 8, cudaMemcpyHostToDevice, st));
-            forward_solve(ctx, Wk, n, n, x, n, 1);
-            backward_solve_vec(ctx, Wk, n, n, x);
-            int hflag = 0;
-            SPG_CUDA_C(cudaMemcpyAsync(hx.data(), x, (size_t) n * 8, cudaMemcpyDeviceToHost, st));
-            SPG_CUDA_C(cudaMemcpyAsync(&hflag, flag, 4, cudaMemcpyDeviceToHost, st));
-            SPG_CUDA_C(cudaStreamSynchronize(st));
-            const bool ok2 = hflag == 0;
-            // update (push / oplus)
-            if(ok2)
-                for(int v = 0; v < dg.nV; v++)
-                    if(pos[v] >= 0) oplus_flat(dg.dim, &dg.poses[(size_t) v * dg.P], &hx[pos[v]]);
-            SPG_CUDA_C(push_poses());
-            double tempChi = 0;
-            SPG_TRY(chi2_only(&tempChi));
-            if(!ok2) tempChi = std::numeric_limits<double>::max();
-            rho = chi - tempChi;
-            double scale = 0; // computeScale: sum x_j (lambda x_j + b_j), b = -g
-            for(int q = 0; q < n; q++) scale += hx[q] * (lambda * hx[q] - hg[q]);
-            scale += 1e-3;
-            rho /= scale;
-            if(rho > 0 && std::isfinite(tempChi)) { // last step was good
-                double alpha = 1.0 - std::pow(2 * rho - 1, 3);
-                alpha = std::min(alpha, 2.0 / 3.0);
-                lambda *= std::max(1.0 / 3.0, alpha);
-                ni = 2;
-                chi = tempChi;
-            } else {
-                lambda *= ni;
-                ni *= 2;
-                dg.poses = saved; // pop
-                SPG_CUDA_C(push_poses());
-                if(!std::isfinite(lambda)) break;
-            }
-            qmax++;
-            trials_total++;
-        } while(rho < 0 && qmax < 10);
-        iters++;
-        if(qmax == 10 || rho == 0 || !std::isfinite(lambda)) terminated = true;
     }
-    SPG_CUDA_C(cudaStreamSynchronize(st));
+    const size_t nn = (size_t) std::max(n, 1);
+    SPG_CUDA_C(dg_.reserve(nn * 8));
+    SPG_CUDA_C(dsc.reserve(64));
+    if(!dense) {
+        SPG_TRY(build_bsr(dg, pos, n, bsr));
+        sparse.reset(new SparseSystem(ctx, dg, arr, bsr, n));
+        SPG_TRY(sparse->reserve());
+    }
+    SPG_TRY(upload(ctx, dg, pos, arr, dense ? nullptr : &bsr));
+    LinearSystem &sys = dense ? static_cast<LinearSystem &>(*dense) : static_cast<LinearSystem &>(*sparse);
+    LmResult res;
+    SPG_TRY(levenberg_marquardt(ctx, dg, arr, pos, n, max_iterations, sys, static_cast<double *>(dg_.p),
+                                static_cast<double *>(dsc.p), res));
+    const bool used_dense = dense != nullptr;
+    const int64_t cg_iterations = sys.cg_iterations;
+    const double cg_max_rel = sys.cg_max_rel_residual;
     cleanup();
 #undef SPG_CUDA_C
 #undef SPG_TRY
@@ -848,13 +1157,16 @@ spg_status spg_graph_optimize(spg_ctx *ctx, spg_graph *gr, const int32_t *fixed_
     }
     G.version++;
     if(stats) {
-        stats->iterations = iters;
-        stats->trials = trials_total;
+        stats->iterations = res.iterations;
+        stats->trials = res.trials;
         stats->dimensions = n;
-        stats->chi2_initial = chi_initial;
-        stats->chi2_final = chi;
-        stats->lambda_final = lambda;
-        stats->terminated = terminated ? 1 : 0;
+        stats->chi2_initial = res.chi2_initial;
+        stats->chi2_final = res.chi2;
+        stats->lambda_final = res.lambda;
+        stats->terminated = res.terminated ? 1 : 0;
+        stats->solver = used_dense ? SPG_SOLVER_DENSE_CHOLESKY : SPG_SOLVER_SPARSE_PCG;
+        stats->cg_iterations = (int32_t) std::min<int64_t>(cg_iterations, std::numeric_limits<int32_t>::max());
+        stats->cg_max_rel_residual = cg_max_rel;
     }
     return SPG_OK;
 }
